@@ -2,6 +2,7 @@
 """Benchmark of the Asyrp hot path: 256x256 images/sec for a complete 40-step Asyrp edit trajectory.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--workload NAME]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -19,9 +20,13 @@ Prints ONE JSON line (rank 0):
                  sustained bf16 cuBLAS peak; `traffic` is read from the committed ncu capture under profiles/
   parity         engine vs the REFERENCE's own output (tests/golden/, written by tests/golden/make_golden.py) on the
                  same weights / x_T / noise, for this workload
-  cpu_baseline   the reference's own CPU code (baseline/_ref, staged by scripts/stage_reference.py; falls back to the
+  cpu_baseline   the reference's own CPU code (oracle/_ref, staged by oracle/stage_reference.py; falls back to the
                  restatement oracle/ = kind "port") on a bounded sample, on the host's cores
   eager_gpu_baseline  the reference's own modules + denoising_step in eager PyTorch (TF32 default) on the same B200
+
+`--dump-outputs DIR` writes what the device-timed path computed in its last step: DIR/x0.npy, the float32 x_0 of the
+whole job (every rank's batch shard, in rank order, gathered to rank 0).  Weights, x_T and the pre-drawn noise are
+seeded, so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` times the reference's CPU implementation: a "step" there is a bounded sample (one edit reverse step
 + one non-edit reverse step at B=1, scaled x n_edit / x n_plain to a trajectory), `ms_per_step` is the measured time of
@@ -40,7 +45,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 GOLD = os.path.join(ROOT, "tests", "golden")
 
 METRIC = "256x256 images/sec, 40-step Asyrp edit"
@@ -124,17 +129,31 @@ def build_model(family, key, device, ckpt=None, seed=1234):
     return model.to(device), delta
 
 
+def dump_outputs(d, arrays, max_bytes=64 * 10**6, seed=1234):
+    """--dump-outputs: each tensor as d/<name>.npy in float32, max_bytes in all; a tensor over its share keeps a seeded
+    sample of its leading-axis rows (ascending), the same rows in every run with the same arguments"""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    share = max_bytes // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            rows = max(1, share // (a.nbytes // a.shape[0]))
+            a = a[np.sort(np.random.default_rng(seed).choice(a.shape[0], rows, replace=False))]
+        np.save(os.path.join(d, f"{name}.npy"), a)
+
+
 def f_img(key, steps, n_edit):
     e, d, dl = FLOPS[key]
     return (steps * (e + d) + n_edit * (d + dl)) * 1e9
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# the reference itself (baseline/_ref): CPU arm, CPU baseline, eager-GPU baseline
+# the reference itself (oracle/_ref): CPU arm, CPU baseline, eager-GPU baseline
 # ---------------------------------------------------------------------------------------------------------------
 def reference_model(family, key, state_dict, device):
     """the reference's own UNet class (models/ddpm/diffusion.py:327, improved_ddpm/script_util.py:102) holding
-    `state_dict`; None when baseline/_ref has not been staged"""
+    `state_dict`; None when oracle/_ref has not been staged"""
     if not os.path.isdir(os.path.join(REF_DIR, "models")):
         return None, None
     if REF_DIR not in sys.path:
@@ -194,7 +213,7 @@ def cpu_setup(family, key, ckpt, traj_steps):
         def run(only):
             return reference_trajectory(ref, du, x, seq, seq_next, betas, logvar, family == "adm", only=only)[1]
         kind = "reference"
-    else:  # baseline/_ref not staged: the restatement (oracle/) — the one other place bench.py may execute oracle/
+    else:  # oracle/_ref not staged: the restatement (oracle/) — the one other place bench.py may execute oracle/
         from oracle import adm as oa, ddpm as od, sampler as osmp
         if family == "ddpm":
             fwd = lambda *a, **k: od.ddpm_forward(sd, od.CELEBA_CFG, *a, **k)  # noqa: E731
@@ -243,7 +262,7 @@ def cpu_sample(run, kind, seq, traj_steps, reps=1):
         if te + tp < sum(best):
             best = (te, tp)
     traj_s = n_edit * best[0] + (traj_steps - n_edit) * best[1]
-    what = "the reference's own denoising_step + UNet (baseline/_ref)" if kind == "reference" else \
+    what = "the reference's own denoising_step + UNet (oracle/_ref)" if kind == "reference" else \
         "fp32 torch CPU restatement of the reference (oracle/)"
     return {"value": 1.0 / traj_s, "unit": "img/s", "cores": torch.get_num_threads(), "kind": kind,
             "sample": f"B=1: 1 edit reverse step ({best[0]:.2f}s) + 1 non-edit reverse step ({best[1]:.2f}s) of the "
@@ -305,7 +324,7 @@ def eager_gpu(family, key, ckpt, batch, traj_steps, dev, reps=2, golden=None):
     torch.cuda.empty_cache()
     return {"value": round(batch / best, 3), "unit": "img/s", "batch": batch, "s_per_trajectory": round(best, 3),
             "parity_vs_cpu_reference": ref_parity,
-            "how": "baseline/_ref modules + utils.diffusion_utils.denoising_step in the save_image loop "
+            "how": "oracle/_ref modules + utils.diffusion_utils.denoising_step in the save_image loop "
                    "(diffusion_latent.py:499-520), eager PyTorch on cuda:0, fp32 tensors, "
                    f"cudnn.allow_tf32={torch.backends.cudnn.allow_tf32}, matmul.allow_tf32="
                    f"{torch.backends.cuda.matmul.allow_tf32}; the reference always runs both decoders (34.4 vs the "
@@ -366,7 +385,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write x_0 of the last timed step as DIR/x0.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 arm")
     family, key, batch, traj_steps, ckpt, golden = WORKLOADS[args.workload]
     batch = args.batch or batch
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
@@ -412,7 +437,7 @@ def main():
         cb = {"value": value, "unit": "img/s", "cores": torch.get_num_threads(), "kind": kind,
               "sample": f"each step = 1 edit reverse step ({te:.2f}s) + 1 non-edit reverse step ({tp:.2f}s) at B=1, "
                         f"scaled x{n_edit}/x{traj_steps - n_edit} to the {traj_steps}-step trajectory; "
-                        f"{'the reference own code from baseline/_ref' if kind == 'reference' else 'oracle/ port'}, "
+                        f"{'the reference own code from oracle/_ref' if kind == 'reference' else 'oracle/ port'}, "
                         f"{torch.get_num_threads()} threads"}
         line = {"impl": "reference", "metric": METRIC, "value": value, "unit": "img/s", "n_gpus": args.gpus,
                 "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1000.0 * timed / args.steps,
@@ -452,7 +477,9 @@ def main():
     x_host = torch.randn(batch, 3, 256, 256, generator=g).pin_memory()
     out_host = torch.empty_like(x_host).pin_memory()
     x_dev = x_host.to(dev)
-    noise = torch.randn(sch.n_stochastic, batch, 3, 256, 256, device=dev)
+    # seeded like x_T, on a generator of its own: the same noise in every run, whatever else draws random numbers
+    noise = torch.randn(sch.n_stochastic, batch, 3, 256, 256, device=dev,
+                        generator=torch.Generator(device=dev).manual_seed(1234 + rank))
 
     def barrier():
         if dist is not None:
@@ -479,6 +506,14 @@ def main():
     ms_per_step = ms.item() / args.steps
     value = batch * args.gpus / (ms_per_step / 1000.0)
     launches = eng.last_launches * args.steps
+    if args.dump_outputs:
+        x0 = out_dev
+        if dist is not None:  # what a caller of the batch-sharded job receives: every rank's shard, in rank order
+            shards = [torch.empty_like(out_dev) for _ in range(world)]
+            dist.all_gather(shards, out_dev)
+            x0 = torch.cat(shards)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"x0": x0})
 
     # ---- end to end through the runner API: pinned host x_T -> device -> trajectory -> pinned host x_0
     for _ in range(2):

@@ -1,10 +1,10 @@
-"""Generate the golden fixtures under tests/golden/ by running the REFERENCE'S OWN modules (imported from
-/root/reference, which only exists in the build container) on the synthetic weights of oracle/synth.py.
+"""Generate the golden fixtures under tests/golden/ by running the REFERENCE'S OWN modules (imported from the
+reference checkout, oracle/stage_reference.reference_dir()) on the synthetic weights of oracle/synth.py.
 
     python tests/golden/make_golden.py [--full] [--traj celeba16,afhq,imagenet]
 
-The fixtures pin the oracle (tests/test_oracle.py, CPU) and are what the CUDA engine is compared with on the GPU
-box, where /root/reference does not exist.  Nothing here is imported by the product package.
+The fixtures pin the oracle (tests/test_oracle.py, CPU) and are what the CUDA engine is compared with on the GPU,
+where the tests never read the reference itself.  Nothing here is imported by the product package.
 
 Fixtures (npz, fp32):
   ddpm_mini.npz / adm_mini.npz      full tensors of reduced configurations: plain forward, Asyrp forward
@@ -33,8 +33,9 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
 sys.path.insert(0, ROOT)
+from oracle.stage_reference import reference_dir  # noqa: E402
+REF = reference_dir()
 sys.path.insert(0, REF)
 
 from oracle import adm as o_adm, ddpm as o_ddpm, sampler as o_smp, synth  # noqa: E402

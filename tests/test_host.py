@@ -62,7 +62,8 @@ def test_param_inventory_matches_oracle_inventory():
 
 def test_module_state_dict_and_delta_checkpoint_format():
     """same keys as the reference modules; a Δh checkpoint {"0": layer_0.state_dict()} loads with all keys matched
-    (diffusion_latent.py:674-676).  Uses a shipped checkpoint when the reference tree is present."""
+    (diffusion_latent.py:674-676).  Uses the reference's shipped 'smiling' DeltaBlock (tests/golden/checkpoint/: its
+    "0" entry, tensor for tensor)."""
     from asyrp_official_b200 import modules, synthetic
     from asyrp_official_b200.configs import load_config
     m = modules.DDPM(load_config("celeba.yml"))
@@ -71,14 +72,11 @@ def test_module_state_dict_and_delta_checkpoint_format():
     assert keys == {"conv1.weight", "conv1.bias", "temb_proj.weight", "temb_proj.bias", "norm2.weight", "norm2.bias",
                     "conv2.weight", "conv2.bias"}
     v0 = m._version
-    ck = "/root/reference/checkpoint/smiling_LC_CelebA_HQ_t999_ninv40_ngen40_0.pth"
-    if os.path.exists(ck):
-        sd = torch.load(ck, map_location="cpu", weights_only=True)["0"]
-        res = m.layer_0.load_state_dict(sd)
-        assert not res.missing_keys and not res.unexpected_keys
-        assert torch.equal(m.layer_0.conv1.weight, sd["conv1.weight"])
-    else:
-        m.layer_0.load_state_dict({k: torch.zeros_like(v) for k, v in m.layer_0.state_dict().items()})
+    ck = os.path.join(ROOT, "tests", "golden", "checkpoint", "smiling_LC_CelebA_HQ_t999_ninv40_ngen40_0.pth")
+    sd = torch.load(ck, map_location="cpu", weights_only=True)["0"]
+    res = m.layer_0.load_state_dict(sd)
+    assert not res.missing_keys and not res.unexpected_keys
+    assert torch.equal(m.layer_0.conv1.weight, sd["conv1.weight"])
     assert m._version > v0  # engine weights are re-packed after any load_state_dict
     a = modules.i_DDPM("AFHQ")
     a.setattr_layers(1)
@@ -142,16 +140,16 @@ def test_config_and_cli_surface(tmp_path, monkeypatch):
 
 
 def test_runner_host_logic():
-    """sequences, hs_coeff scaling (diffusion_latent.py:626,654,659) and LPIPS-table t_edit lookup"""
+    """sequences, hs_coeff scaling (diffusion_latent.py:626,654,659) and LPIPS-table t_edit lookup on the CelebA-HQ
+    tables the reference ships (utils/celeba_LPIPS_distance_{x0_t,x}.tsv, stored under tests/golden/lpips/)"""
     from asyrp_official_b200.configs import load_config
     from asyrp_official_b200.diffusion_latent import Asyrp
     a = argparse.Namespace(user_defined_t_edit=None, user_defined_t_addnoise=None, clip_cosine=0.8, config="celeba.yml",
-                           lpips_table_dir="/root/reference/utils", add_noise_from_xt=True)
+                           lpips_table_dir=os.path.join(ROOT, "tests", "golden", "lpips"), add_noise_from_xt=True)
     r = Asyrp(a, load_config("celeba"), device="cpu")
     assert r.betas.dtype == torch.float32 and r.logvar.shape == (1000,)
-    if os.path.isdir(a.lpips_table_dir):
-        r.set_t_edit_t_addnoise(LPIPS_th=0.33, LPIPS_addnoise_th=1.2)
-        assert 400 <= r.t_edit <= 560 and r.t_addnoise == 167  # SURVEY.md Appendix D
+    r.set_t_edit_t_addnoise(LPIPS_th=0.33, LPIPS_addnoise_th=1.2)
+    assert 400 <= r.t_edit <= 560 and r.t_addnoise == 167  # SURVEY.md Appendix D
     a2 = argparse.Namespace(user_defined_t_edit=500, user_defined_t_addnoise=200)
     r2 = Asyrp(a2, load_config("celeba"), device="cpu")
     r2.set_t_edit_t_addnoise()
@@ -261,23 +259,40 @@ def test_schedule_sample_type_dt_lambda_and_key(mode):
     assert torch.allclose(ref, mine, rtol=0, atol=1e-6) and s.c1 == 0.0
 
 
-def test_reference_staging_script(tmp_path):
-    """scripts/stage_reference.py copies the reference's hot-path sources verbatim into a git-ignored directory
-    (only where /root/reference exists, i.e. in the build container)"""
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("stage_reference", os.path.join(ROOT, "scripts", "stage_reference.py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    assert "baseline/_ref/" in open(os.path.join(ROOT, ".gitignore")).read()
-    if not os.path.isdir("/root/reference"):
-        assert mod.stage("/root/reference", str(tmp_path / "x"), quiet=True) is False
-        return
-    assert mod.stage("/root/reference", str(tmp_path / "ref"), quiet=True)
-    for rel in ("utils/diffusion_utils.py", "models/ddpm/diffusion.py", "models/improved_ddpm/unet.py",
-                "models/guided_diffusion/unet.py", "configs/celeba.yml",
-                "checkpoint/smiling_LC_CelebA_HQ_t999_ninv40_ngen40_0.pth"):
-        a, b = os.path.join("/root/reference", rel), os.path.join(str(tmp_path / "ref"), rel)
-        assert open(a, "rb").read() == open(b, "rb").read(), rel
+def test_reference_staging_script(tmp_path, monkeypatch):
+    """oracle/stage_reference.py copies the reference's hot-path sources verbatim into a git-ignored directory, on a
+    stand-in checkout with the reference's layout; the checkout is $ASYRP_REFERENCE_DIR, else the default location"""
+    from oracle import stage_reference as mod
+    assert "oracle/_ref/" in open(os.path.join(ROOT, ".gitignore")).read()
+    assert mod.DST == os.path.join(ROOT, "oracle", "_ref")
+    monkeypatch.delenv("ASYRP_REFERENCE_DIR", raising=False)
+    monkeypatch.setattr(mod, "REFERENCE", str(tmp_path / "missing"))
+    assert mod.stage(None, str(tmp_path / "x"), quiet=True) is False
+    assert mod.stage(str(tmp_path / "missing"), str(tmp_path / "x"), quiet=True) is False
+    assert not (tmp_path / "x").exists()
+    src = tmp_path / "src"
+    files = {rel: f"{rel}\n".encode() * 3 for rel in (
+        "utils/diffusion_utils.py", "models/ddpm/diffusion.py", "models/improved_ddpm/unet.py",
+        "models/guided_diffusion/unet.py", "configs/celeba.yml", *(f"checkpoint/{c}" for c in mod.CKPTS))}
+    skipped = ("utils/celeba_LPIPS_distance_x.tsv", "models/__pycache__/m.cpython-312.pyc", "checkpoint/other_0.pth",
+               "main.py")
+    for rel in (*files, *skipped):
+        (src / rel).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel).write_bytes(files.get(rel, b"x"))
+    for how in ("default", "env"):
+        dst = tmp_path / f"ref_{how}"
+        (dst / "models").mkdir(parents=True)
+        (dst / "models" / "stale.py").write_text("")  # an earlier staging's leftovers are replaced
+        if how == "default":
+            monkeypatch.setattr(mod, "REFERENCE", str(src))
+        else:
+            monkeypatch.setattr(mod, "REFERENCE", str(tmp_path / "missing"))
+            monkeypatch.setenv("ASYRP_REFERENCE_DIR", str(src))
+        assert mod.stage(dst=str(dst), quiet=True)
+        staged = {os.path.relpath(os.path.join(d, f), dst) for d, _, fs in os.walk(dst) for f in fs}
+        assert staged == set(files)
+        for rel, data in files.items():
+            assert (dst / rel).read_bytes() == data, rel
 
 
 def test_engine_numerics_emulation_switches():
