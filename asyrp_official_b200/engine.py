@@ -32,8 +32,8 @@ FUSE_MIN_H = int(os.environ.get("ASYRP_FUSE_MIN_H", "16"))
 # of 315 launches per edit evaluation, non-conv time 1.04 -> 0.68 ms — but the conv kernels pay more than that back
 # (per-tile group statistics on the transform warps' critical path, 64-bit atomics in every epilogue): measured
 # 34.2 -> 32.0 img/s (DDPM b16), 35.8 -> 33.7 (AFHQ b8), 5.45 -> 5.17 (ImageNet b4).  Off by default; the path is
-# complete and covered by tests (test_groupnorm_finalised_inside_the_consumer_conv, and the whole GPU suite passes
-# with it on).
+# complete and covered by tests (test_groupnorm_finalised_inside_the_consumer_conv, and tests/test_plan_replay_gpu.py
+# replays every launch of the four bench plans built with it on).
 GN_FOLD = os.environ.get("ASYRP_GN_FOLD", "0") in ("1", "2")
 GN_FOLD_PRODUCERS_ONLY = os.environ.get("ASYRP_GN_FOLD", "0") == "2"  # diagnostic: atomics on, consumers use tables
 # ResBlock identity skips x + h ride conv2's K loop as an identity weight block (C extra MACs per output, exact: fp16 x
